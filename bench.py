@@ -53,6 +53,9 @@ def parse():
     ap.add_argument("--no-torch-cuda-baseline", action="store_true")
     ap.add_argument("--ref-full", action="store_true", help="torch-CUDA baseline: run all DDIM steps for every precision mode")
     ap.add_argument("--dump-ops", default=None, help="write the per-op timing table of one UNet evaluation to this CSV")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the waveforms [clips, 1, samples] of the last timed step to DIR/wave.npy (float32; the leading clips "
+                         "that fit in 64 MB): the inputs depend only on the arguments, so two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -334,6 +337,20 @@ def kernel_pass(eng, peaks: dict, dump=None):
                 unet_eval_ms_eager=round(total, 3), lane_rows=pl.meta.get("Bt"))
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, wave, rank):
+    """Rank 0 writes the waveforms of the whole batch (as many leading clips as fit in DUMP_BYTES) as float32."""
+    if rank != 0:
+        return
+    import numpy as np
+    row = wave[0].numel() * 4
+    w = wave[:max(1, DUMP_BYTES // row)].float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "wave.npy"), w)
+
+
 def main():
     a = parse()
     if a.impl == "reference":
@@ -402,7 +419,13 @@ def main():
     if rank == 0:
         clocks.start()
     # (1) device-resident: conditioning (and input audio) already in HBM, waveform left in HBM
-    t_dev = timed(lambda i: generate(42 + i, cond_d, unc_d, wav_d), a.steps)
+    last = {}
+
+    def dev_step(i):
+        last["wave"] = generate(42 + i, cond_d, unc_d, wav_d)           # the engine's waveform slot: rewritten by the next call
+    t_dev = timed(dev_step, a.steps)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, parallel.all_gather_rows(last["wave"], Bg), rank)
 
     # (2) end to end through the public seams: host conditioning / audio -> ... -> waveform in pinned host memory
     def e2e_step(i):

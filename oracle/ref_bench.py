@@ -5,9 +5,9 @@ Two back ends, in order of preference:
 
 * ``kind == "reference"``: the UNMODIFIED reference modules -- ``UNetModel`` (openaimodel.py:837-885), ``Decoder``
   (model.py:653-686), ``Generator`` (hifigan/models.py:149-165) driven by the reference ``DDIMSampler``
-  (ddim.py:166-355, two ``apply_model`` calls per step as ddim.py:293-296) -- imported from ``baseline/_ref``
-  (``pip install --no-deps --target baseline/_ref`` of /root/reference, git-ignored, travels to the GPU box) or from
-  ``/root/reference`` in the build container, with the package ``__init__`` files bypassed (oracle/ref_loader.py).
+  (ddim.py:166-355, two ``apply_model`` calls per step as ddim.py:293-296) -- imported from ``$ALDM_REFERENCE_ROOT`` or
+  from ``baseline/_ref`` (``pip install --no-deps --target baseline/_ref`` of the reference, git-ignored), with the package
+  ``__init__`` files bypassed (oracle/ref_loader.py).  Only paths the caller names or inside the tree are searched.
 * ``kind == "port"``: oracle/functional.py, the torch restatement pinned against those modules by the fixtures.
 
 Both run the seeded synthetic checkpoint / conditioning of SURVEY.md 8d on the device they are given.
@@ -31,7 +31,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _locate_reference() -> Optional[str]:
-    for cand in (os.environ.get("ALDM_REFERENCE_ROOT"), os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
+    for cand in (os.environ.get("ALDM_REFERENCE_ROOT"), os.path.join(ROOT, "baseline", "_ref")):
         if cand and os.path.isdir(os.path.join(cand, "audioldm2", "latent_diffusion")):
             return cand
     return None

@@ -10,10 +10,47 @@ from audioldm2_b200 import synth
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SAMPLER_SEED = 42          # pipeline.py:185 default seed
+MAX_BYTES = 950_000        # every fixture file stays below 1 MB
+BLOCK = 1024               # elements per kept block of a thinned tensor
 
 
 def load(name: str) -> dict:
     return torch.load(os.path.join(HERE, name + ".pt"), map_location="cpu", weights_only=True)
+
+
+def _cols(blocks: torch.Tensor, n: int) -> torch.Tensor:
+    cols = (blocks[:, None] * BLOCK + torch.arange(BLOCK)).reshape(-1)
+    return cols[cols < n]
+
+
+def thin(d: dict, seed: int = 0) -> dict:
+    """A fixture that would exceed MAX_BYTES keeps, of every float tensor of 64 Ki elements or more, the same seeded
+    random subset of BLOCK-element blocks in each row (leading dimension): stored as [rows, kept elements], with the
+    block indices under ``<key>_blocks``.  Tests compare through ``pick``."""
+    size = lambda ks: sum(d[k].numel() * d[k].element_size() for k in ks)
+    tensors = [k for k, v in d.items() if torch.is_tensor(v)]
+    big = [k for k in tensors if d[k].is_floating_point() and d[k].numel() >= 1 << 16]
+    if size(tensors) <= MAX_BYTES or not big:
+        return d
+    frac = (MAX_BYTES - 4096 * len(d) - (size(tensors) - size(big))) / size(big)     # 4 KB of archive overhead per entry
+    g = torch.Generator().manual_seed(seed)
+    out = dict(d)
+    for k in big:
+        x = d[k].reshape(d[k].shape[0], -1)
+        nb = -(-x.shape[1] // BLOCK)
+        blocks = torch.randperm(nb, generator=g)[:int(nb * frac)].sort().values
+        out[k] = x[:, _cols(blocks, x.shape[1])].contiguous()
+        out[k + "_blocks"] = blocks
+    return out
+
+
+def pick(g: dict, key: str, x: torch.Tensor) -> torch.Tensor:
+    """The elements of ``x`` that fixture ``g`` stores for ``key``: all of them, or those ``thin`` kept."""
+    blocks = g.get(key + "_blocks")
+    if blocks is None:
+        return x
+    x = x.reshape(x.shape[0], -1)
+    return x[:, _cols(blocks, x.shape[1]).to(x.device)]
 
 
 def latent(cfg: dict, B: int, seed: int = 3) -> torch.Tensor:

@@ -13,6 +13,8 @@ by ``tests/golden/cases.py`` so only the outputs are stored.
 from __future__ import annotations
 
 import argparse
+import ast
+import json
 import os
 import sys
 import time
@@ -32,7 +34,7 @@ from tests.golden import cases                  # noqa: E402
 
 def _save(name, d):
     path = os.path.join(HERE, name + ".pt")
-    torch.save({k: (v.contiguous() if torch.is_tensor(v) else v) for k, v in d.items()}, path)
+    torch.save(cases.thin({k: (v.contiguous() if torch.is_tensor(v) else v) for k, v in d.items()}), path)
     print(f"wrote {path} ({os.path.getsize(path) / 1e3:.0f} KB)")
 
 
@@ -158,6 +160,19 @@ def gen_stft(R, name, n_fft, hop, n_mels, sr, fmin, fmax, n_samples):
     _save(name, dict(logmel=mel, mag_l2=torch.linalg.norm(mag)))
 
 
+def gen_signatures(name):
+    """Argument names and the source text of the defaults of the public pipeline functions (pipeline.py)."""
+    src = open(os.path.join(ref_loader.REF_ROOT, "audioldm2", "pipeline.py")).read()
+    out = {n.name: dict(args=[a.arg for a in n.args.args], defaults=[ast.get_source_segment(src, d) for d in n.args.defaults])
+           for n in ast.parse(src).body
+           if isinstance(n, ast.FunctionDef) and n.name in ("build_model", "text_to_audio", "super_resolution_and_inpainting")}
+    path = os.path.join(HERE, name + ".json")
+    with open(path, "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print(f"wrote {path}")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--only", default=None)
@@ -196,6 +211,7 @@ def main():
         "vocoder_48k_full": lambda: gen_vocoder(R, "vocoder_48k_full", m48, 1, 1024),
         "unet_large_full": lambda: gen_unet(R, "unet_large_full", large, 1),
         "stft_48k": lambda: gen_stft(R, "stft_48k", 2048, 480, 256, 48000, 20, 24000, 491520),
+        "pipeline_signatures": lambda: gen_signatures("pipeline_signatures"),
     }
     for k, fn in jobs.items():
         if a.only and k != a.only:

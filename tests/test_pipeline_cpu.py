@@ -37,14 +37,15 @@ def test_signatures_match_reference(name):
 
 
 def test_signatures_against_reference_source_when_present():
+    """REF_SIGNATURES against the signatures parsed from the reference's pipeline.py (tests/golden/make_golden.py)."""
     import ast
-    path = "/root/reference/audioldm2/pipeline.py"
-    if not os.path.exists(path):
-        pytest.skip("reference tree absent (GPU box)")
-    for node in ast.parse(open(path).read()).body:
-        if isinstance(node, ast.FunctionDef) and node.name in REF_SIGNATURES:
-            assert [a.arg for a in node.args.args] == REF_SIGNATURES[node.name][0]
-            assert [ast.literal_eval(d) for d in node.args.defaults] == REF_SIGNATURES[node.name][1]
+    import json
+    with open(os.path.join(cases.HERE, "pipeline_signatures.json")) as f:
+        ref = json.load(f)
+    assert sorted(ref) == sorted(REF_SIGNATURES)
+    for name, sig in ref.items():
+        assert sig["args"] == REF_SIGNATURES[name][0]
+        assert [ast.literal_eval(d) for d in sig["defaults"]] == REF_SIGNATURES[name][1]
 
 
 def test_package_exports():
